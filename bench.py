@@ -1,6 +1,6 @@
 """bench.py - utterances/s of the speaker-conditioned mask-estimation forward pass on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp16_f8c|fp16x3|bf16x3|fp16|bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp16_f8c|fp16x3|bf16x3|fp16|bf16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one pass of the hot path (CNN -> BiLSTM -> FC -> sigmoid mask -> mask * spectrogram)
@@ -112,6 +112,28 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each [B, ...] device output as out_dir/<name>.npy (float32).  When all of them together exceed DUMP_BYTES, the same
+    evenly spaced utterances (always the first and the last) are kept from each, so two builds run with the same arguments can be
+    compared output for output."""
+    B = next(iter(arrays.values())).shape[0]
+    keep = min(B, DUMP_BYTES // sum(a[0].numel() * 4 for a in arrays.values()))
+    if keep < 1:
+        raise SystemExit(f"--dump-outputs: one utterance's outputs exceed {DUMP_BYTES} bytes")
+    idx = np.linspace(0, B - 1, keep).round().astype(np.int64)
+    sel = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    shapes = {}
+    for name, a in arrays.items():
+        out = a.index_select(0, sel).float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+        shapes[name] = list(out.shape)
+    return {"dir": out_dir, "shapes": shapes, "utterances": "all" if keep == B else idx.tolist()}
+
+
 def _usable_cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -194,7 +216,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip every secondary block (training, config 2, baselines)")
     ap.add_argument("--no-train", action="store_true", help="skip the config-4 training block")
     ap.add_argument("--train-batch", type=int, default=256, help="config 4: utterances per GPU to try first (halved until it fits)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write mask.npy and masked.npy of the last timed step to DIR (rank 0; "
+                                                           "evenly spaced whole utterances when all of them exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -242,12 +268,15 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps):
+    def timed(fn, steps, keep_last=None):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
-        for _ in range(steps):
-            fn()
+        for i in range(steps):
+            if keep_last is not None and i == steps - 1:
+                keep_last.append(fn())
+            else:
+                fn()        # earlier outputs are dropped at once, so the allocator serves every step from the same blocks
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
@@ -300,12 +329,15 @@ def main():
     if rank == 0:
         sampler.start()
     eng.set_profiling(True)
-    local_ms = timed(lambda: eng.forward(x, emb, precision=prec, want_masked=True), args.steps)
+    last = [] if args.dump_outputs else None
+    local_ms = timed(lambda: eng.forward(x, emb, precision=prec, want_masked=True), args.steps, keep_last=last)
     kernel_ms = {}
     for name, ms in eng.profile_read():           # per-kernel times of the last timed step
         kernel_ms[name] = kernel_ms.get(name, 0.0) + ms
     launches_per_step = eng.last_launch_count()
     eng.set_profiling(False)
+    dumped = dump_outputs(args.dump_outputs, dict(zip(("mask", "masked"), last[0]))) if last and rank == 0 else None
+    last = None
     value, dev_ms = vdist.aggregate_throughput(B * args.steps, local_ms, dist, dev)
     # ---- end to end through the host-buffer plugin call ("e2e"): every step copies its inputs from pinned
     # host memory, runs the forward and copies mask + masked back.  The serving form of the call is
@@ -419,6 +451,8 @@ def main():
                 "kernel_ms_last_step": {k: round(v, 4) for k, v in kernel_ms.items()},
                 "gflop_per_utt": {k: v / 1e9 for k, v in fl.items()},
                 "tflops_total_algorithmic": fl["total"] * value / 1e12}
+        if dumped:
+            line["dumped_outputs"] = dumped
 
     # free the inference buffers before the secondary blocks
     del eng, x, emb, xh, eh, mask_h, masked_h, ref32, got

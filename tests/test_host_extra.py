@@ -1,5 +1,6 @@
 """Host-side logic of the section-8f components that needs no GPU: state_dict layout of the speaker encoder, batch grouping
 of the evaluation driver, and the torch criterion against the loss oracle."""
+import json
 import os
 import shutil
 import subprocess
@@ -11,8 +12,6 @@ import torch
 from oracle import loss_oracle
 from voicesplit_b200 import evaluate, losses, synth
 from voicesplit_b200.speaker_encoder import SpeakerEncoder
-
-CKPT = "/root/reference/notebooks/embedder.pt"
 
 
 def test_speaker_encoder_state_dict_layout():
@@ -32,10 +31,14 @@ def test_speaker_encoder_state_dict_layout():
     enc.load_state_dict({k: torch.from_numpy(v) for k, v in synth.make_encoder_state_dict(0).items()}, strict=True)
 
 
-@pytest.mark.skipif(not os.path.isfile(CKPT), reason="reference checkpoint not present")
 def test_speaker_encoder_loads_the_reference_checkpoint_unchanged():
+    # key / shape / dtype of every tensor in the reference's GE2E checkpoint (notebooks/embedder.pt, 48 MB), recorded by
+    # tests/golden/make_reference_checks_golden.py; a strict load checks exactly these
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_layouts.json")) as f:
+        layout = json.load(f)["embedder_checkpoint"]
+    ckpt = {k: torch.zeros(shape, dtype=getattr(torch, dtype)) for k, shape, dtype in layout}
     enc = SpeakerEncoder(40, 3, 768, 80, 40)                      # the notebook's positional arguments (:88)
-    missing = enc.load_state_dict(torch.load(CKPT, map_location="cpu"), strict=True)
+    missing = enc.load_state_dict(ckpt, strict=True)
     assert not missing.missing_keys and not missing.unexpected_keys
 
 
